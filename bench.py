@@ -10,6 +10,7 @@ library (C ABI, include/agrep_b200.h).
 
   python bench.py --gpus N --steps K --warmup W            our arm (one rank per GPU under torchrun)
   python bench.py --impl reference ...                      the reference's own CPU scan on the host cores
+  python bench.py ... --dump-outputs DIR                    also write what the last timed step returned, as DIR/*.npy
 
 Prints ONE JSON line (rank 0).  `value` = corpus bytes / device time (inputs resident in HBM);
 `e2e` = the same scan through agb_scan_host() on pinned HOST buffers, H2D and result D2H inside the timing;
@@ -191,6 +192,27 @@ class ClockSampler:
                 "samples": len(sm), "source": "nvidia-smi -lms 100"}
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, n_matched, records=None):
+    """What a caller of the timed path receives from its last step, as float64 .npy files (byte offsets up to 2^53 are exact):
+    n_matched.npy = [matching records], records.npy = their ordered (begin, end) rows.  A list larger than DUMP_LIMIT is cut to
+    a fixed sample of rows (seed 0, kept in order), records_rows.npy says which.  The corpus, and so the answer, depends only
+    on the arguments and AGB_BENCH_GIB: two builds can be compared file by file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "n_matched.npy"), np.array([n_matched], dtype=np.float64))
+    if records is None:
+        return
+    if records.nbytes > DUMP_LIMIT - (1 << 20):
+        keep = (DUMP_LIMIT - (1 << 20)) // (records.shape[1] * 8 + 8)
+        rows = np.sort(np.random.default_rng(0).choice(records.shape[0], keep, replace=False))
+        records = records[rows]
+        np.save(os.path.join(out_dir, "records_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "records.npy"), records.astype(np.float64))
+
+
 # ----------------------------------------------------------------------------------------------------
 def run_reference(args):
     """The reference's own CPU implementation of the path, all host threads: one unmodified `agrep -c -n -2`
@@ -239,6 +261,8 @@ def run_reference(args):
             matched = step()
         dt = (time.perf_counter() - t0) / max(1, args.steps)
         val = total / dt / 1e9
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, matched)
         sample = ("%d shards x %d MiB = %.1f GiB of the same synthetic corpus per step (a bounded sample of the %.0f GiB workload; GB/s is "
                   "size-normalised), one `agrep -V0 -c -n -%d` process per usable host core" % (cores, shard >> 20, total / (1 << 30), TOTAL_GIB, K))
         print(json.dumps({
@@ -397,7 +421,10 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
     if args.impl == "reference":
         return run_reference(args)
@@ -501,6 +528,9 @@ def main():
     launches = L.agb_kernel_launches() - launches0
     clocks = sampler.stop() if rank == 0 else None
     matched_total = gathered
+    if args.dump_outputs and rank == 0:
+        # before anything else writes into recs; with N > 1 the gathered list of the whole corpus is on every rank
+        dump_outputs(args.dump_outputs, int(res.n_matched), recs[:gathered, :2].cpu().numpy())
 
     # ---- end to end through the host-buffer entry point (pinned host memory, H2D + result D2H inside the timing)
     n_e2e = min(int(E2E_GIB * (1 << 30)), n_local - HR) // PAGE * PAGE

@@ -1,10 +1,12 @@
 """The drop-in proof: the reference program linked against libagrepb200_dropin.so (oracle/_ref/agrep_dropin:
 the reference's own main(), option parser, exec() and output(); only bitap/asearch/asearch0/asearch1/sgrep/
 fill_buf come from this repo and run on the GPU) must print byte-for-byte what the unmodified reference
-(oracle/_ref/agrep) prints.  Both binaries are built here by oracle/Makefile and travel to the GPU box."""
-import os, subprocess, tempfile
+(oracle/_ref/agrep) prints.  oracle/Makefile builds both where the reference sources are; without them the drop-in cases
+skip.  The stand-alone command line (agrep-b200) is checked against the reference's stdout stored in
+tests/golden/reference_runs.json (tests/_reference.py), so it runs on any checkout."""
+import hashlib, os, subprocess, tempfile
 import pytest
-import _corpus
+import _corpus, _reference
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -14,19 +16,20 @@ DROP = os.path.join(ROOT, "oracle", "_ref", "agrep_dropin")
 from _corpus import overlap_text
 
 
+def texts():
+    return (("a.txt", _corpus.make_text(3000, seed=11)), ("b.txt", _corpus.make_text(2000, seed=12, trailing_newline=False)),
+            ("para.txt", _corpus.make_text(2500, seed=13, paragraphs=True)),
+            ("small.txt", _corpus.make_text(600, seed=14)),       # < 48 KiB: no block artefacts in -b (SURVEY 8c(1))
+            ("semi.txt", _corpus.make_text(300, seed=15).replace(b"\n", b";").replace(b"the", b"Hello", 30).replace(b"and", b"xhello", 10) + b"last hello there"),   # (not "hello" at the very end: bm()'s sentinel copy of the pattern behind the text makes -w see a letter there)
+            ("blank.txt", b"\n" * 3000 + b"one the two\n" + b"\n" * 3000 + b"x\n\n\ny"),   # more than half of the bytes close a record
+            ("aba.txt", overlap_text("aba", 5)))      # a delimiter that overlaps itself, with chains ("abababa")
+
+
 @pytest.fixture(scope="module")
 def files():
-    if not (os.path.exists(REF) and os.path.exists(DROP)):
-        pytest.skip("oracle/_ref binaries not built")
     d = tempfile.mkdtemp(prefix="agb_dropin_")
     paths = {}
-    for name, data in (("a.txt", _corpus.make_text(3000, seed=11)), ("b.txt", _corpus.make_text(2000, seed=12, trailing_newline=False)),
-                       ("para.txt", _corpus.make_text(2500, seed=13, paragraphs=True)),
-                       ("small.txt", _corpus.make_text(600, seed=14)),       # < 48 KiB: no block artefacts in -b (SURVEY 8c(1))
-                       ("semi.txt", _corpus.make_text(300, seed=15).replace(b"\n", b";").replace(b"the", b"Hello", 30).replace(b"and", b"xhello", 10) + b"last hello there"),   # (not "hello" at the very end: bm()'s sentinel copy of the pattern behind the text makes -w see a letter there)
-                       ("blank.txt", b"\n" * 3000 + b"one the two\n" + b"\n" * 3000 + b"x\n\n\ny"),   # more than half of the bytes close a record
-                       ("aba.txt", overlap_text("aba", 5))):      # a delimiter that overlaps itself, with chains ("abababa")
-
+    for name, data in texts():
         paths[name] = os.path.join(d, name)
         open(paths[name], "wb").write(data)
     yield paths
@@ -35,9 +38,14 @@ def files():
     os.rmdir(d)
 
 
-def run(binary, args):
-    p = subprocess.run([binary] + args, capture_output=True, timeout=120, stdin=subprocess.DEVNULL)
+def run(binary, args, cwd=None):
+    p = subprocess.run([binary] + args, capture_output=True, timeout=120, stdin=subprocess.DEVNULL, cwd=cwd)
     return p.returncode, p.stdout, p.stderr
+
+
+def needs_dropin(*binaries):
+    if not all(os.path.exists(b) for b in binaries):
+        pytest.skip("the drop-in binaries link the reference's own objects: oracle/_ref is built only where its sources are")
 
 
 CASES = [
@@ -79,6 +87,7 @@ CASES = [
 
 @pytest.mark.parametrize("args,names", CASES)
 def test_same_stdout_as_reference(files, args, names):
+    needs_dropin(REF, DROP)
     fl = [files[n] for n in names]
     r = run(REF, ["-V0"] + args + fl)
     d = run(DROP, ["-V0"] + args + fl)
@@ -94,13 +103,13 @@ CLI_CASES = [c for c in CASES if not any(a in ("-L2", "-s") or a.startswith("-S"
 
 @pytest.mark.parametrize("args,names", CLI_CASES)
 def test_standalone_cli_prints_what_the_reference_prints(files, args, names):
-    """agrep-b200 (agrep_b200/csrc/agrep_main.c): our own main() + output() restatement over the engine."""
-    if not os.path.exists(CLI):
-        pytest.skip("agrep-b200 not built")
-    fl = [files[n] for n in names]
-    r = run(REF, args + fl)                      # default verbosity: with the "Grand Total" line
-    d = run(CLI, args + fl)
-    assert d[1] == r[1]
+    """agrep-b200 (agrep_b200/csrc/agrep_main.c): our own main() + output() restatement over the engine.  Both run where
+    the files are, on their bare names (names are part of the output): exit code, length and sha-256 of stdout."""
+    data = dict(texts())
+    summary = lambda rc, out, err: [rc, len(out), hashlib.sha256(out).hexdigest()]
+    r = _reference.answer("rc_stdout_size_sha256", args, [(n, data[n]) for n in names], summary)   # default verbosity: with the "Grand Total" line
+    d = summary(*run(CLI, args + names, cwd=os.path.dirname(files[names[0]])))
+    assert d[1:] == r[1:]
     assert d[0] == r[0]
 
 
@@ -115,8 +124,7 @@ def test_memory_mode_through_the_dropin(files, args, name):
     """memagrep() (agrep.c:3282; scan loop bitap.c:309-446): the reference's in-memory entry point with the scan objects
     replaced by the drop-in layer (fd == -1: the caller's buffer is scanned, no delimiter is appended behind it, so an
     undelimited last record is not reported -- by -c either) prints and returns what the unmodified one does."""
-    if not (os.path.exists(MEM) and os.path.exists(MEMDROP)):
-        pytest.skip("oracle/_ref memagrep drivers not built")
+    needs_dropin(MEM, MEMDROP)
     r = run(MEM, [files[name], "-V0"] + args)
     d = run(MEMDROP, [files[name], "-V0"] + args)
     assert d[1] == r[1] and d[0] == r[0]
@@ -130,8 +138,7 @@ def test_three_gib_file_streams_through_the_dropin(tmp_path):
     import resource, shutil, sys
     sys.path.insert(0, ROOT)
     import agrep_b200 as ag
-    if not (os.path.exists(REF) and os.path.exists(DROP)):
-        pytest.skip("oracle/_ref binaries not built")
+    needs_dropin(REF, DROP)
     base = "/dev/shm" if os.path.isdir("/dev/shm") and shutil.disk_usage("/dev/shm").free > (5 << 30) else str(tmp_path)
     if shutil.disk_usage(base).free < (4 << 30):
         pytest.skip("no room for a 3 GiB file")

@@ -1,31 +1,25 @@
-"""Pins oracle/agrep_oracle.c against the UNMODIFIED reference built from /root/reference by
-oracle/Makefile (oracle/_ref/agrep).  Skipped when the reference binary is absent (GPU box keeps the
-prebuilt one, so this also runs there).  Reference invocations follow SURVEY.md 8(c):
+"""Pins oracle/agrep_oracle.c against the UNMODIFIED reference (oracle/_ref/agrep, built by oracle/Makefile), through
+its answers stored in tests/golden/reference_runs.json (tests/_reference.py).  Reference invocations follow SURVEY.md 8(c):
 k>0 automaton forced with -n, unit-cost asearch1 with -S1, simple literals via sgrep/bm."""
-import os, random, re, subprocess, tempfile
+import random, re
 import pytest
-import _oracle, _corpus
+import _oracle, _corpus, _reference
 
 
-def run_ref(ref, args, data):
-    with tempfile.NamedTemporaryFile(suffix=".txt", delete=False) as f:
-        f.write(data)
-        path = f.name
-    try:
-        p = subprocess.run([ref, "-V0"] + args + [path], capture_output=True, timeout=120)
-        return p.stdout
-    finally:
-        os.unlink(path)
+def ref(what, args, data, read):
+    return _reference.answer(what, ["-V0"] + args, [("text.txt", data)], read)
 
 
-def ref_count(ref, args, data):
-    out = run_ref(ref, ["-c"] + args, data).strip()
-    return int(out) if out else 0
+def ref_count(args, data):
+    return ref("count", ["-c"] + args, data, lambda rc, out, err: int(out.strip()) if out.strip() else 0)
 
 
-def ref_ordinals(ref, args, data):
-    out = run_ref(ref, ["-n"] + args, data)
-    return [int(m.group(1)) for m in re.finditer(rb"^(\d+): ", out, re.M)]
+def ordinals(out, pattern=rb"^(\d+): "):
+    return [int(m.group(1)) for m in re.finditer(pattern, out, re.M)]
+
+
+def ref_ordinals(args, data):
+    return ref("ordinals", ["-n"] + args, data, lambda rc, out, err: ordinals(out))
 
 
 TEXT = _corpus.make_text(4000, seed=12345)
@@ -61,39 +55,33 @@ CASES = [
 
 @pytest.mark.parametrize("pattern,okw,rargs", CASES)
 @pytest.mark.parametrize("which", ["nl", "nonl"])
-def test_automaton_matches_reference(ref_agrep, pattern, okw, rargs, which):
-    if not ref_agrep:
-        pytest.skip("reference binary not built")
+def test_automaton_matches_reference(pattern, okw, rargs, which):
     data = TEXT if which == "nl" else TEXT_NONL
     a = _oracle.compile(pattern, width=32, **okw)
     cnt, recs = _oracle.scan(a, data)
-    assert cnt == ref_count(ref_agrep, ["-n"] + rargs + [pattern], data)
+    assert cnt == ref_count(["-n"] + rargs + [pattern], data)
     # -n prints j-1 (agrep.c:3878)
-    assert [r[2] - 1 for r in recs] == ref_ordinals(ref_agrep, rargs + [pattern], data)
+    assert [r[2] - 1 for r in recs] == ref_ordinals(rargs + [pattern], data)
 
 
 @pytest.mark.parametrize("pattern,k", [("win", 0), ("because each", 2), ("state", 1)])
-def test_paragraph_records(ref_agrep, pattern, k):
-    if not ref_agrep:
-        pytest.skip("reference binary not built")
+def test_paragraph_records(pattern, k):
     a = _oracle.compile(pattern, width=32, k=k, linenum=1, wordbound=1, delim="$$")
     cnt, recs = _oracle.scan(a, PARA)
-    assert cnt == ref_count(ref_agrep, ["-n", "-w", "-d", "$$", "-%d" % k, pattern] if k else ["-n", "-w", "-d", "$$", pattern], PARA)
+    assert cnt == ref_count(["-n", "-w", "-d", "$$", "-%d" % k, pattern] if k else ["-n", "-w", "-d", "$$", pattern], PARA)
 
 
 @pytest.mark.parametrize("pattern,kw,rargs", [
     ("the", {}, []), ("The", {}, []), ("government", {}, []), ("the", dict(wordbound=1), ["-w"]),
     ("each", dict(nocase=1), ["-i"]), ("zzzz", {}, [])])
 @pytest.mark.parametrize("which", ["nl", "nonl"])
-def test_sgrep_bm_counts(ref_agrep, pattern, kw, rargs, which):
+def test_sgrep_bm_counts(pattern, kw, rargs, which):
     """config 1: `agrep -c the` goes through sgrep()->bm() (case-insensitive substring, once per line)."""
-    if not ref_agrep:
-        pytest.skip("reference binary not built")
     data = TEXT if which == "nl" else TEXT_NONL
     a = _oracle.compile(pattern, **kw)
     assert a.engine == 4
     cnt, _ = _oracle.scan(a, data, want_records=False)
-    assert cnt == ref_count(ref_agrep, rargs + [pattern], data)
+    assert cnt == ref_count(rargs + [pattern], data)
 
 
 @pytest.mark.parametrize("pattern,delim,kw,rargs", [
@@ -101,47 +89,39 @@ def test_sgrep_bm_counts(ref_agrep, pattern, kw, rargs, which):
     ("state", ";", dict(nocase=1), ["-i"]), ("because each", "%", {}, []),
     ("homogeneous approximate matching", ";", {}, []),          # > 20 characters: monkey() instead of bm() (sgrep.c:407-442, 1540)
 ])
-def test_sgrep_keeps_its_engine_under_d(ref_agrep, pattern, delim, kw, rargs):
+def test_sgrep_keeps_its_engine_under_d(pattern, delim, kw, rargs):
     """checksg() does not look at -d: a simple literal at k=0 still goes to sgrep()/bm() -- ASCII case folded whatever -i
     says -- and bm() cuts the records with backward_/forward_delimiter() (sgrep.c:775-795)."""
-    if not ref_agrep:
-        pytest.skip("reference binary not built")
     body = TEXT[:30000].replace(b"\n", delim.encode(), 400).replace(b"the", b"Hello", 40).replace(b"and", b"xhello", 20)
     for data in (b"Hello world;foo bar;HELLO again;nothing".replace(b";", delim.encode()), body, delim.encode() + body, body + delim.encode()):
         a = _oracle.compile(pattern, delim=delim, **kw)
         assert a.engine == 4
         cnt, _ = _oracle.scan(a, data, want_records=False)
-        assert cnt == ref_count(ref_agrep, rargs + ["-d", delim, pattern], data), (pattern, delim, data[:40])
+        assert cnt == ref_count(rargs + ["-d", delim, pattern], data), (pattern, delim, data[:40])
 
 
 @pytest.mark.parametrize("pattern", ["the of and to in that is was he for", "homogeneous approximate matching", "governmental homogeneous"])
-def test_sgrep_long_literals_take_monkey(ref_agrep, pattern):
+def test_sgrep_long_literals_take_monkey(pattern):
     """m > 20 (LONG_EXAC): the reference runs monkey() instead of bm() (sgrep.c:407-442, 1540-1834); same record semantics"""
-    if not ref_agrep:
-        pytest.skip("reference binary not built")
     data = TEXT + (b"xx " + pattern.encode() + b" yy\n") * 3 + pattern.upper().encode() + b"\n" + TEXT[:5000]
     a = _oracle.compile(pattern)
     assert a.engine == 4 and a.litlen > 20
     cnt, _ = _oracle.scan(a, data, want_records=False)
-    assert cnt >= 4 and cnt == ref_count(ref_agrep, [pattern], data)
+    assert cnt >= 4 and cnt == ref_count([pattern], data)
 
 
-def test_latin1_fold_is_the_table_the_reference_ends_up_with(ref_agrep):
+def test_latin1_fold_is_the_table_the_reference_ends_up_with():
     """-i at k=0 reads bytes through LUT[] (bitap.c:171) = CP[ISO-8859-1].lower_1 with the metasymbol bytes put back to
     themselves (agrep.c:2835-2848): 0xC9 folds to 0xE9, but 0x83 does not fold to 'f', 0x8f not to 0x86, 0x99 not to 0x94"""
-    if not ref_agrep:
-        pytest.skip("reference binary not built")
     data = b"\x83ood one\nfood two\nab\x99cd\nab\x94cd\ncaf\xc9 x\ncaf\xe9 y\nq\x8fq\nq\x86q\n"
     for pat in (b"food", b"b\x94c", b"caf\xe9", b"q\x86q", b"\x83ood", b"b\x99c"):
         a = _oracle.compile(pat, k=0, linenum=1, nocase=1)
         cnt, recs = _oracle.scan(a, data)
-        assert [r[2] - 1 for r in recs] == ref_ordinals(ref_agrep, ["-i", pat], data), pat
+        assert [r[2] - 1 for r in recs] == ref_ordinals(["-i", pat], data), pat
 
 
-def test_random_differential(ref_agrep):
+def test_random_differential():
     """SURVEY appendix A differential driver: random substrings with 0-2 edits, k in 1..3, -n forced."""
-    if not ref_agrep:
-        pytest.skip("reference binary not built")
     rnd = random.Random(2024)
     lines = TEXT.decode().split("\n")
     for trial in range(40):
@@ -156,7 +136,7 @@ def test_random_differential(ref_agrep):
             continue
         a = _oracle.compile(pat, width=32, k=k, linenum=1)
         cnt, recs = _oracle.scan(a, TEXT)
-        assert [r[2] - 1 for r in recs] == ref_ordinals(ref_agrep, ["-%d" % k, pat], TEXT), (pat, k)
+        assert [r[2] - 1 for r in recs] == ref_ordinals(["-%d" % k, pat], TEXT), (pat, k)
 
 
 def test_pattern_too_long_matches_reference_limit():
@@ -167,12 +147,10 @@ def test_pattern_too_long_matches_reference_limit():
     _oracle.compile("a" * 40, width=64, k=1, linenum=1)
 
 
-def test_random_metachar_differential(ref_agrep):
+def test_random_metachar_differential():
     """random patterns with classes, '.', '#', <>, ',' and ';', anchors, under -i/-w/-v/-p/-S2 and user delimiters, on a
     text shorter than one 48 KiB block (no block artefacts): ordinals of the matching lines (newline records), counts
     (user delimiters: their records are not one per output line).  Cases the reference refuses are skipped."""
-    if not ref_agrep:
-        pytest.skip("reference binary not built")
     base = _corpus.make_text(400, seed=5)
     words = [w for w in base.decode().split() if w.isalpha()]
     rnd = random.Random(31)
@@ -207,20 +185,17 @@ def test_random_metachar_differential(ref_agrep):
             continue
         cnt, recs = _oracle.scan(a, data)
         if "delim" in kw:
-            out = run_ref(ref_agrep, ["-c", "-n"] + args + [pat], data).strip()
-            if out.isdigit():
-                assert int(out) == cnt, (pat, args)
+            out = ref("count_if_accepted", ["-c", "-n"] + args + [pat], data,
+                      lambda rc, out, err: int(out.strip()) if out.strip().isdigit() else None)
+            if out is not None:
+                assert out == cnt, (pat, args)
                 compared += 1
             continue
-        with tempfile.NamedTemporaryFile(suffix=".txt", delete=False) as f:
-            f.write(data)
-        try:
-            p = subprocess.run([ref_agrep, "-V0", "-n"] + args + [pat, f.name], capture_output=True, timeout=120)
-        finally:
-            os.unlink(f.name)
-        if p.returncode == 255 or p.stderr.strip():
+        out = ref("ordinals_if_accepted", ["-n"] + args + [pat], data,
+                  lambda rc, out, err: None if rc == 255 or err.strip() else ordinals(out))
+        if out is None:
             continue
-        assert [r[2] - 1 for r in recs] == [int(m.group(1)) for m in re.finditer(rb"^(\d+): ", p.stdout, re.M)], (pat, args)
+        assert [r[2] - 1 for r in recs] == out, (pat, args)
         compared += 1
     assert compared > 100
 
@@ -231,37 +206,33 @@ from _corpus import overlap_text
 @pytest.mark.parametrize("delim", ["aba", "abab", "=-=", "e e", "xyx"])
 @pytest.mark.parametrize("pattern,kw,rargs", [("state", dict(k=1, linenum=1), ["-1"]), ("e", dict(k=0, linenum=1), []),
                                               ("world", dict(k=0, linenum=1, inverse=1), ["-v"])])
-def test_self_overlapping_delimiters(ref_agrep, delim, pattern, kw, rargs):
+def test_self_overlapping_delimiters(delim, pattern, kw, rargs):
     """a delimiter that overlaps itself: the automaton takes occurrences from the left and drops those that share a byte with
     one it took (asearch.c:55-57, 175-186) -- count and ordinals of the restatement against the reference binary"""
-    if not ref_agrep:
-        pytest.skip("reference binary not built")
     for seed in (3, 4):
         data = overlap_text(delim, seed)
         for d in (data, delim.encode() + data, data + delim.encode(), data[:-len(delim)] + delim.encode()[:-1]):
             a = _oracle.compile(pattern, delim=delim, **kw)
             cnt, recs = _oracle.scan(a, d)
             assert cnt > 3
-            assert cnt == ref_count(ref_agrep, ["-n"] + rargs + ["-d", delim, pattern], d), (delim, pattern)
-            out = run_ref(ref_agrep, ["-n"] + rargs + ["-d", delim, pattern], d)
+            assert cnt == ref_count(["-n"] + rargs + ["-d", delim, pattern], d), (delim, pattern)
+            out = ref("record_numbers", ["-n"] + rargs + ["-d", delim, pattern], d, lambda rc, out, err: ordinals(out, rb"(\d+): "))
             # (with a user delimiter -n prints j itself: the record count starts one lower, bitap.c:151-156 / agrep.c:3878)
-            assert [r[2] for r in recs] == [int(m.group(1)) for m in re.finditer(rb"(\d+): ", out)], (delim, pattern)
+            assert [r[2] for r in recs] == out, (delim, pattern)
 
 
 @pytest.mark.parametrize("pattern,kw,rargs", [("because each", dict(k=2, linenum=1), ["-2"]), ("state", dict(k=0, linenum=1), []),
                                               ("gov[ea]rnment", dict(k=1, linenum=1), ["-1"]), ("world", dict(k=1, linenum=1, wordbound=1), ["-1", "-w"])])
-def test_inverse_count_is_records_minus_matches(ref_agrep, pattern, kw, rargs):
+def test_inverse_count_is_records_minus_matches(pattern, kw, rargs):
     """what the device's complement count rests on (scan.cu complement_usable): under -v every newline record either matches
     or does not, so `-c -v` = records - `-c`, with records = newlines + one for an unterminated last line -- checked on the
     reference binary itself and on the restatement, for texts with blank lines, without a final newline, starting with
     newlines, ending in a match"""
-    if not ref_agrep:
-        pytest.skip("reference binary not built")
     body = TEXT[:40000]
     for data in (body, body[:-1], b"\n\n" + body, body.replace(b"the\n", b"the\n\n\n", 40), body + b"because each", body + b"\n\n\n", b"\n", b"x"):
         records = data.count(b"\n") + (0 if data.endswith(b"\n") else 1)
-        pos = ref_count(ref_agrep, ["-n"] + rargs + [pattern], data)
-        inv = ref_count(ref_agrep, ["-n", "-v"] + rargs + [pattern], data)
+        pos = ref_count(["-n"] + rargs + [pattern], data)
+        inv = ref_count(["-n", "-v"] + rargs + [pattern], data)
         assert inv == records - pos, (pattern, len(data), inv, records, pos)
         a = _oracle.compile(pattern, inverse=1, **kw)
         assert _oracle.scan(a, data, want_records=False)[0] == inv
