@@ -326,7 +326,10 @@ __global__ void __launch_bounds__(ORD_THREADS) k_delim_count(const OrdParams P)
 }
 
 /* the tile counts from block counts that stage 1 already took (front.cu, COUNT): 64 blocks per tile, plus the
- * delimiter appended at EOF, which no block of the text has seen (position n; L = 1 on this path) */
+ * delimiter appended at EOF, which no block of the text has seen (position n; L = 1 on this path).  That one is added
+ * to the tile sum only, never written back to its block: a rerun of the record stage (stages_after_front) runs this
+ * kernel again over the same block counts and must count it once.  No reader needs it in the block -- k_ordinals and
+ * k_shard_aux sum only the blocks below their own, and the EOF block is the last one that holds text. */
 __global__ void __launch_bounds__(256) k_ord_tiles(const OrdParams P, uint64_t n_tiles)
 {
 	/* a warp per tile: its 64 block counts are 128 consecutive bytes */
@@ -337,8 +340,8 @@ __global__ void __launch_bounds__(256) k_ord_tiles(const OrdParams P, uint64_t n
 	const uint64_t b = t * 64 + 2 * lane, eof_blk = P.n / ORD_BLOCK;
 	const uint32_t two = *reinterpret_cast<const uint32_t *>(P.blocks + b);
 	uint32_t lo = two & 0xFFFFu, hi = two >> 16;
-	if (b == eof_blk) { lo += 1; P.blocks[b] = (uint16_t)lo; }
-	if (b + 1 == eof_blk) { hi += 1; P.blocks[b + 1] = (uint16_t)hi; }
+	if (b == eof_blk) lo += 1;
+	if (b + 1 == eof_blk) hi += 1;
 	const uint32_t sum = __reduce_add_sync(0xffffffffu, lo + hi);
 	if (lane == 0) P.tiles[t] = sum;
 }
